@@ -9,11 +9,14 @@ device-resident replay shard (sum-tree descent + IS weights + 7-frame window gat
 fused IQN loss, backward, (gradient all-reduce when N > 1), Adam, priority update of the sampled leaves.
 N > 1 is the data-parallel learner of config 5 (512 transitions per GPU, weak scaling).
 
-Timing: W untimed warm-up steps, then `--blocks` regions of EXACTLY K steps each, every one bracketed by barrier +
-torch.cuda.synchronize(), CUDA events on the launching stream, max over ranks; the headline is the median block.  A
-`sustained` leg (>= 3 s of steps, clocks sampled) and the end-to-end leg (pinned host batches, H2D / D2H inside the timed
-region) follow.  Inputs are larger than L2: every step draws a fresh prioritized minibatch from a multi-GB replay shard
-and streams > 1 GB of activations.  Also in the line: rooflines of the hidden products (tensor), the embedding producer,
+Timing: W untimed warm-up steps, then ONE region of exactly K timed steps, bracketed by barrier +
+torch.cuda.synchronize(), CUDA events on the launching stream, max over ranks (`--blocks R` times R such regions and
+reports the median).  The last timed step starts from the seeded network, optimiser and replay state (restored untimed),
+and `--dump-outputs DIR` writes what it returned (sampled tree indices and per-transition losses, rank 0) as
+DIR/<name>.npy, so two builds run with the same arguments can be compared output for output.  An optional
+`--sustained-seconds` leg (clocks sampled) and the end-to-end leg (K steps, pinned host batches, H2D / D2H inside the
+timed region) follow.  Inputs are larger than L2: every step draws a fresh prioritized minibatch from a multi-GB replay
+shard and streams > 1 GB of activations.  Also in the line: rooflines of the hidden products (tensor), the embedding producer,
 the conv trunk and the loss kernel (HBM), the Rainbow-only (C51, configs[2]) leg, and the CPU port timed on the host cores.
 `--topology apex` (N >= 2) runs configs[3] instead: 1 learner rank + N-1 actor GPUs with sharded replay.
 Prints ONE JSON line on rank 0.
@@ -159,6 +162,12 @@ def run_ours(args):
     parallel.make_data_parallel(learner)
     mem = ReplayMemory(a, None)
     fill_replay(mem, args.replay_capacity, dev, 1000 + rank)
+    # the device state one step leaves for the next (noise and sampling draws follow the step count), as seeded; it is
+    # restored before the last timed step because the gradients' fp32 atomics make trajectories drift apart run to run
+    # and prioritized sampling turns that drift into different minibatches
+    seeded = (learner.online_net._flat, learner.optimiser._exp_avg, learner.optimiser._exp_avg_sq,
+              mem.transitions.tree, mem.transitions.max_priority)
+    seeded = [(t, t.clone()) for t in seeded]
 
     def barrier():
         if world > 1:
@@ -166,7 +175,7 @@ def run_ours(args):
         torch.cuda.synchronize()
 
     def step():
-        return learner.learn_and_update(mem)[1]
+        return learner.learn_and_update(mem)
 
     # ---- pass 1 (eager, not the headline): per-entry-point device times for the roofline section
     for _ in range(3):
@@ -202,18 +211,28 @@ def run_ours(args):
     clocks = ClockSampler(local)
     clocks.start()
     # `blocks` timed regions of EXACTLY args.steps steps each (barrier + synchronize on both sides, CUDA events on the
-    # launching stream, max over ranks); the headline is the MEDIAN block, the spread is reported beside it
+    # launching stream, max over ranks); the headline is the MEDIAN block, the spread is reported beside it.  The last
+    # step of a region starts from the seeded state, so what it returns is the same in every run with these arguments;
+    # the restoring copies lie between two event pairs and are not timed.
+    e2, e3 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     block_ms = []
     for _ in range(max(1, args.blocks)):
         barrier()
         e0.record()
-        for _ in range(args.steps):
-            loss = step()
+        for _ in range(args.steps - 1):
+            step()
         e1.record()
+        for t, t0 in seeded:
+            t.copy_(t0)
+        e2.record()
+        idxs, loss = step()
+        e3.record()
         barrier()
-        block_ms.append(parallel.allreduce_max(e0.elapsed_time(e1), dev))
+        block_ms.append(parallel.allreduce_max(e0.elapsed_time(e1) + e2.elapsed_time(e3), dev))
     launches = launches_per_step * args.steps          # kernels executed in ONE timed region (graph replays them)
     clk = clocks.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, {"tree_idxs": idxs.cpu().double().numpy(), "loss": loss.cpu().float().numpy()})
     ms = float(np.median(block_ms))
     ms_per_step = ms / args.steps
     value = world * 1000.0 / ms_per_step
@@ -359,6 +378,14 @@ def run_ours(args):
     finish(world)
 
 
+def dump_outputs(directory, arrays):
+    """Write each host array as `directory`/<name>.npy (float32 or float64; tree indices are exact in float64)."""
+    os.makedirs(directory, exist_ok=True)
+    for name, a in arrays.items():
+        assert a.dtype in (np.float32, np.float64), (name, a.dtype)
+        np.save(os.path.join(directory, name + ".npy"), a)
+
+
 def finish(world):
     """End of a run: all ranks meet once more, then leave WITHOUT tearing NCCL down.  destroy_process_group() (and the
     interpreter's own teardown) can block forever when CUDA graphs that captured collectives are still alive (seen on
@@ -430,7 +457,7 @@ def c51_leg(dev, args):
             learner.learn_and_update(mem)
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-    n = max(args.steps, 20)
+    n = args.steps
     e0.record()
     for _ in range(n):
         loss = learner.learn_and_update(mem)[1]
@@ -680,11 +707,17 @@ def main():
     ap.add_argument("--actor-envs", type=int, default=128, help="apex: environments per actor GPU")
     ap.add_argument("--actor-buffer", type=int, default=200, help="apex: steps per actor buffer flush (reference: 1000)")
     ap.add_argument("--acts-per-step", type=int, default=1, help="apex: batched acting iterations per learner step")
-    ap.add_argument("--blocks", type=int, default=5, help="timed regions of --steps steps each; the median is the headline")
-    ap.add_argument("--sustained-seconds", type=float, default=3.0, help="length of the sustained leg (0 = skip)")
+    ap.add_argument("--blocks", type=int, default=1, help="timed regions of --steps steps each; the median is the headline")
+    ap.add_argument("--sustained-seconds", type=float, default=0.0, help="length of the sustained leg (0 = skip)")
     ap.add_argument("--no-graph", action="store_true", help="eager launches instead of CUDA-graph replay")
     ap.add_argument("--max-seconds", type=int, default=900, help="watchdog: abort the process after this long")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the outputs of the last timed learner step (rank 0) as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be >= 1")
+    if args.dump_outputs and (args.impl != "ours" or args.topology != "dp"):
+        ap.error("--dump-outputs applies to the data-parallel learner (--impl ours --topology dp)")
     watchdog(args.max_seconds)
     if args.impl == "reference":
         run_reference(args)

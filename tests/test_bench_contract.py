@@ -37,3 +37,30 @@ def test_reference_arm_line(capsys, monkeypatch):
     monkeypatch.setenv("RANK", "1")
     bench.run_reference(args)
     assert capsys.readouterr().out == ""
+
+
+def test_dump_outputs_files(tmp_path):
+    import numpy as np
+    import pytest
+    import bench
+    d = str(tmp_path / "out")
+    idx, loss = np.arange(512, dtype=np.float64) + 2 ** 40, np.linspace(0, 1, 512, dtype=np.float32)
+    bench.dump_outputs(d, {"tree_idxs": idx, "loss": loss})
+    assert sorted(os.listdir(d)) == ["loss.npy", "tree_idxs.npy"]
+    assert np.array_equal(np.load(os.path.join(d, "tree_idxs.npy")), idx)
+    got = np.load(os.path.join(d, "loss.npy"))
+    assert got.dtype == np.float32 and np.array_equal(got, loss)
+    with pytest.raises(AssertionError):
+        bench.dump_outputs(d, {"tree_idxs": idx.astype(np.int64)})
+
+
+def test_bench_argument_checks(monkeypatch, tmp_path):
+    import pytest
+    import bench
+    for argv in (["--steps", "0"], ["--impl", "reference", "--dump-outputs", str(tmp_path)],
+                 ["--gpus", "2", "--topology", "apex", "--dump-outputs", str(tmp_path)]):
+        monkeypatch.setattr(sys, "argv", ["bench.py", *argv])
+        with pytest.raises(SystemExit) as e:
+            bench.main()
+        assert e.value.code == 2, argv
+    assert not os.listdir(tmp_path)
