@@ -726,6 +726,19 @@ __global__ void unpermute_add_kernel(int Cout, int K, const float* __restrict__ 
   dw[(long)c * K + perm[kp]] += dwp[idx];
 }
 
+// Weight image of the strip data gradient (TC_DGRAD operand B, (Cout, t*t*Kc) row-major, Kc = s*s*Cin):
+//   wd[co, (dy*t + dx)*Kc + n] = w[co, c, s*dy + sy, s*dx + sx],   n = (sy, c, sx), sx fastest
+// -- the column order in which the TC_DGRAD epilogue stores din.  w is the (Cout, Cin*KH*KW) bf16 weight.
+__global__ void dgrad_weight_kernel(riqn_conv_geom g, int t, const bf16* __restrict__ w, bf16* __restrict__ wd) {
+  const int s = g.stride, sc = s * g.Cin, Kc = s * sc, K = g.Cin * g.KH * g.KW;
+  const int idx = blockIdx.x * blockDim.x + threadIdx.x;
+  if (idx >= g.Cout * K) return;
+  const int co = idx / K, q = idx - co * K;
+  const int sft = q / Kc, n = q - sft * Kc, dy = sft / t, dx = sft - dy * t;
+  const int sy = n / sc, r = n - sy * sc, c = r / s, sx = r - c * s;
+  wd[idx] = w[(long)co * K + (c * g.KH + s * dy + sy) * g.KW + s * dx + sx];
+}
+
 static int strip_params(const riqn_conv_geom* g, int* t, int* G, int* kc) {
   if (g->KH != g->KW || g->stride < 1 || g->KH % g->stride) return 1;
   *t = g->KH / g->stride;
@@ -780,20 +793,37 @@ RIQN_API int riqn_conv_fwd_strip(const riqn_conv_geom* g, const void* a_hi, cons
 //   dYg (B*G*G, Cout) = dout * (out > 0) on the strip grid;   dbias += column sums
 //   dW'[c, (shift, within)] = sum_m' dYg[m', c] * a_hi[m' + shift offset, within]   (MN-major operands, shifted rows)
 //   dw[c, perm[k']] += wgrad_scale * dW'[c, k']
-//   din += col2im(dYg * W)   (W (Cout, K) as MN-major operand; fused epilogue, pad == 0 only; din may be NULL)
+//   din = sum_shift dYg[m' - shift offset] * Wd_shift   (pad == 0 only; din may be NULL): the forward's shifted-row product
+//        with negative shifts on the same block grid (TC_DGRAD), every din element written once -- no col2im scatter.
+//        Wd is the bf16 weight in (shift, sy, c, sx) column order, built in the front of dwp_scratch before the weight
+//        gradient needs that buffer.
 RIQN_API int riqn_conv_bwd_strip(const riqn_conv_geom* g, const float* dout, const float* out, const void* a_hi,
                                  const void* w_hi, const int* perm, void* dYg, float* dwp_scratch, float* dw, float* dbias,
                                  float* din, float wgrad_scale, void* stream) {
-  riqn::note_launches(din ? 6 : 4);
   cudaStream_t s = (cudaStream_t)stream;
   int t, G, kc;
   if (strip_params(g, &t, &G, &kc) || g->Cout > 64 || g->Cout % 8 || (din && g->pad != 0)) return (int)cudaErrorInvalidValue;
+  // pad == 0: G*stride <= H; a remainder row / column (H - KH not a multiple of the stride) is read by no output
+  const bool margin = din && (G * g->stride != g->H || G * g->stride != g->W);
+  riqn::note_launches(din ? (margin ? 7 : 6) : 4);
   const long Mg = (long)g->B * G * G;
   const int K = g->Cin * g->KH * g->KW;
   const long tiles = (Mg + 63) / 64;
   conv_dy_grid_kernel<<<(unsigned)(tiles < 148 * 4 ? tiles : 148 * 4), 256, 0, s>>>(g->B, g->Cout, g->OH, g->OW, G, dout, out,
                                                                                 (bf16*)dYg, dbias);
   RIQN_LAUNCH_CHECK();
+  if (din) {
+    bf16* wd = reinterpret_cast<bf16*>(dwp_scratch);      // Cout*K bf16 in a buffer of Cout*K floats
+    dgrad_weight_kernel<<<(g->Cout * K + 255) / 256, 256, 0, s>>>(*g, t, (const bf16*)w_hi, wd);
+    RIQN_LAUNCH_CHECK();
+    if (margin) RIQN_CUDA(cudaMemsetAsync(din, 0, sizeof(float) * (size_t)g->B * g->Cin * g->H * g->W, s));
+    TcExtra dg;
+    dg.strip_t = t; dg.strip_G = G; dg.dg_cout = g->Cout;
+    dg.ci_h = g->H; dg.ci_w = g->W; dg.ci_cin = g->Cin; dg.ci_stride = g->stride;
+    const int rc = gemm_bf16_tc((int)Mg, kc * 64, t * t * 64, (const bf16*)dYg, nullptr, wd, nullptr, din, 0, TC_DGRAD,
+                                nullptr, nullptr, nullptr, 1, s, &dg);
+    if (rc) return rc;
+  }
   RIQN_CUDA(cudaMemsetAsync(dwp_scratch, 0, sizeof(float) * g->Cout * K, s));
   TcExtra ex;
   ex.mn_major = 3;
@@ -806,17 +836,6 @@ RIQN_API int riqn_conv_bwd_strip(const riqn_conv_geom* g, const float* dout, con
   if (rc) return rc;
   unpermute_add_kernel<<<(g->Cout * K + 255) / 256, 256, 0, s>>>(g->Cout, K, dwp_scratch, perm, dw);
   RIQN_LAUNCH_CHECK();
-  if (din) {
-    RIQN_CUDA(cudaMemsetAsync(din, 0, sizeof(float) * (size_t)g->B * g->Cin * g->H * g->W, s));
-    TcExtra ci;
-    ci.ohw = G * G;
-    ci.ci_h = g->H; ci.ci_w = g->W; ci.ci_cin = g->Cin; ci.ci_kh = g->KH; ci.ci_kw = g->KW;
-    ci.ci_stride = g->stride; ci.ci_ow = g->OW; ci.ci_oh = g->OH; ci.ci_G = G;
-    ci.mn_major = 2;               // B = the (Cout, K) weight itself, read as an MN-major operand (no transposed copy)
-    rc = gemm_bf16_tc((int)Mg, K, g->Cout, (const bf16*)dYg, nullptr, (const bf16*)w_hi, nullptr, din, K, TC_COL2IM, nullptr,
-                      nullptr, nullptr, 1, s, &ci);
-    if (rc) return rc;
-  }
   return 0;
 }
 

@@ -32,7 +32,7 @@ int gemm_f32(int M, int N, int K, const float* A, long sAm, long sAk, const floa
 
 // ---- tcgen05 / TMA path (gemm_tc.cu) ---------------------------------------------------------------------------
 enum TcEpi { TC_STORE = 0, TC_BIAS_RELU = 1, TC_ATOMIC = 2, TC_NOISY_WGRAD = 3, TC_BIAS_RELU_NCHW = 4, TC_EMBED = 5,
-             TC_COL2IM = 6, TC_CONV = 7 };
+             TC_COL2IM = 6, TC_CONV = 7, TC_DGRAD = 8 };
 
 struct TcExtra {
   int ohw = 1;
@@ -41,14 +41,20 @@ struct TcExtra {
   int batch = 1;
   __nv_bfloat16 *o_hi = nullptr, *o_lo = nullptr, *o_hiT = nullptr, *o_loT = nullptr;
   // TC_COL2IM: row m = (b, oh, ow), column n = (c, kh, kw); C is the NCHW image gradient (pad == 0), accumulated into
-  // (ci_G > 0: rows live on the G x G strip grid, m = (b, gy, gx); only gy < ci_oh, gx < ci_ow are real)
-  int ci_h = 0, ci_w = 0, ci_cin = 0, ci_kh = 0, ci_kw = 0, ci_stride = 0, ci_ow = 0, ci_G = 0, ci_oh = 0;
+  int ci_h = 0, ci_w = 0, ci_cin = 0, ci_kh = 0, ci_kw = 0, ci_stride = 0, ci_ow = 0;
   // Strip convolution (TC_CONV): A is the space-to-depth image (B*G*G rows of strip_kc*64 values); k-block kb reads rows
   // m0 + dy*G + dx (shift = kb / strip_kc = dy*strip_t + dx), columns (kb % strip_kc)*64.  Row m = (b, gy, gx) on the
   // G x G grid is a real output iff gy < cv_oh and gx < cv_ow; C is the NCHW fp32 output (relu(acc + bias)); nx_hi / nx_lo
   // (may be null) receive the bf16 images in the NEXT layer's space-to-depth layout (block edge nx_s, grid nx_G).
   int strip_t = 0, strip_G = 0, strip_kc = 0, cv_oh = 0, cv_ow = 0, nx_s = 0, nx_G = 0;
   __nv_bfloat16 *nx_hi = nullptr, *nx_lo = nullptr;
+  // Strip-convolution data gradient (TC_DGRAD), the same shifted-row product with negative shifts:
+  //   din block row m = (b, gy, gx), column n:   C[m, n] = sum_{shift (dy, dx)} dYg[m - dy*G - dx, :] . Wd[:, shift*N + n]
+  // A = dYg (M, dg_cout) K-major (dg_cout <= 64: k-block kb IS shift kb; rows before the first are TMA zero fill),
+  // B = Wd (dg_cout, strip_t^2 * N) read MN-major, K = strip_t^2 * 64, strip_G = G.  Column n = (sy, c, sx) (sx fastest)
+  // is stored once, without atomics, to the NCHW image C[b, c, gy*s + sy, gx*s + sx] (s = ci_stride, image ci_cin x
+  // ci_h x ci_w with G*s <= ci_h, ci_w; pixels beyond G*s, which no output reads, are not written).
+  int dg_cout = 0;
   // MN-major operands (mn_major bit 0: A is (K, M) row-major, bit 1: B is (K, N) row-major): the reduction index is the
   // ROW, as in a weight gradient dW = dY^T X taken straight from the row-major activations, or a data gradient
   // dX = dY W read from the untransposed weight (mn_major = 2).  NSPLIT 1 only.

@@ -277,7 +277,7 @@ struct alignas(64) TcArgs {
   float alpha;           // TC_ATOMIC: scale applied to the accumulator
   int vec_acc;           // TC_ATOMIC / TC_NOISY_WGRAD: C (out2, eps) rows are 16-byte aligned -> vectorised accumulate
   int ohw;               // TC_BIAS_RELU_NCHW: m = b*ohw + p -> C[(b*N + n)*ohw + p]
-  int ci_h, ci_w, ci_cin, ci_kh, ci_kw, ci_stride, ci_ow, ci_G, ci_oh;   // TC_COL2IM geometry (pad == 0)
+  int ci_h, ci_w, ci_cin, ci_kh, ci_kw, ci_stride, ci_ow;   // TC_COL2IM geometry (pad == 0); TC_DGRAD: image, stride
   const float* feat;     // TC_EMBED: (samples, N) conv features, row m uses feat[m / batch] (batch = rows per sample)
   int batch;
   bf16 *o_hi, *o_lo;     // TC_EMBED: bf16 hi / lo images of the result, row-major (M, N)   (may be null)
@@ -348,6 +348,17 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA_hi, const __grid_constan
           mbar_wait(&empty[stage], phase ^ 1);
           uint8_t* s = smem + stage * Cfg::kStageBytes;
           mbar_expect_tx(&full[stage], Cfg::kStageBytes);
+          if (EPI == TC_DGRAD) {
+            // strip data gradient: k-block kb = shift (dy, dx).  A = dYg rows m0 - dy*G - dx (the first tile's negative
+            // rows are zero fill), B = 64 x 64 slabs of the weight image at column kb*N + n, reduction rows 0..63
+            const int dy = kb / p.strip_t;
+            tma_load_2d(s, &mapA_hi, 0, mt * TBM - dy * p.strip_G - (kb - dy * p.strip_t), &full[stage]);
+#pragma unroll
+            for (int i = 0; i < TBN / 64; ++i)
+              tma_load_2d(s + Cfg::kABytes + i * 8192, &mapB_hi, kb * p.N + nt * TBN + 64 * i, 0, &full[stage]);
+            if (++stage == Cfg::kStages) { stage = 0; phase ^= 1; }
+            continue;
+          }
           if (NSPLIT == 1 && p.mn_major) {
             // MN-major operand ((K, MN) row-major): 64 x 64 boxes, inner coordinate = MN offset, outer = reduction row.
             // bit 0: A, bit 1: B; the other operand (if any) stays K-major.
@@ -416,14 +427,15 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA_hi, const __grid_constan
           tc_fence_after();
           const uint32_t sa = smem_u32(smem + stage * Cfg::kStageBytes);
           const uint32_t sb = sa + Cfg::kOps * Cfg::kABytes;
-          if (NSPLIT == 1 && p.mn_major) {
-            const uint32_t idesc_mn = idesc | ((p.mn_major & 1) ? (1u << 15) : 0u) | ((p.mn_major & 2) ? (1u << 16) : 0u);
+          if (NSPLIT == 1 && (p.mn_major || EPI == TC_DGRAD)) {
+            const int mnm = EPI == TC_DGRAD ? 2 : p.mn_major;   // TC_DGRAD: A K-major, B MN-major
+            const uint32_t idesc_mn = idesc | ((mnm & 1) ? (1u << 15) : 0u) | ((mnm & 2) ? (1u << 16) : 0u);
 #pragma unroll
             for (int k = 0; k < TBK / UMMA_K; ++k) {
               const uint32_t koff_mn = k * (UMMA_K / 8) * 1024;   // MN-major: 16 reduction rows = two 8-row swizzle atoms
               const uint32_t koff_k = k * UMMA_K * 2;             // K-major: bytes inside the 128 B swizzle row
-              const uint64_t da = (p.mn_major & 1) ? umma_desc_mn128(sa + koff_mn) : umma_desc_k128(sa + koff_k);
-              const uint64_t db = (p.mn_major & 2) ? umma_desc_mn128(sb + koff_mn) : umma_desc_k128(sb + koff_k);
+              const uint64_t da = (mnm & 1) ? umma_desc_mn128(sa + koff_mn) : umma_desc_k128(sa + koff_k);
+              const uint64_t db = (mnm & 2) ? umma_desc_mn128(sb + koff_mn) : umma_desc_k128(sb + koff_k);
               umma_bf16(tmem_d, da, db, idesc_mn, (kb > kb0 || k > 0) ? 1u : 0u);
             }
             umma_commit(&empty[stage]);
@@ -533,7 +545,7 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA_hi, const __grid_constan
 #pragma unroll
             for (int j = 0; j < 32; ++j)
               if (n0 + j < p.N) cb[(long)j * p.ohw] = fmaxf(__uint_as_float(v[j]) + p.bias[n0 + j], 0.f);
-          } else if (EPI == TC_EMBED || EPI == TC_COL2IM || EPI == TC_CONV) {
+          } else if (EPI == TC_EMBED || EPI == TC_COL2IM || EPI == TC_CONV || EPI == TC_DGRAD) {
             // handled below with the whole warp
           } else if (!(p.vec_acc && n0 + 32 <= p.N)) {
             float* crow = p.C + (long)m * p.ldc + n0;
@@ -614,18 +626,48 @@ gemm_tc_kernel(const __grid_constant__ CUtensorMap mapA_hi, const __grid_constan
             const int kh = r / p.ci_kw, kw = r - kh * p.ci_kw;
             coff = (c * p.ci_h + kh) * p.ci_w + kw;
           }
-          bool row_ok = m < p.M;
+          const bool row_ok = m < p.M;
           const int mm = row_ok ? m : 0;
-          const int b = mm / p.ohw, pp = mm - b * p.ohw;                 // ohw = G*G on the strip grid
-          const int rw = p.ci_G ? p.ci_G : p.ci_ow;
-          const int oh = pp / rw, ow = pp - oh * rw;
-          if (p.ci_G) row_ok = row_ok && oh < p.ci_oh && ow < p.ci_ow;   // grid rows beyond the real outputs carry zeros
+          const int b = mm / p.ohw, pp = mm - b * p.ohw;
+          const int oh = pp / p.ci_ow, ow = pp - oh * p.ci_ow;
           float* base = p.C + ((long)b * p.ci_cin * p.ci_h + oh * p.ci_stride) * p.ci_w + ow * p.ci_stride;
 #pragma unroll
           for (int j = 0; j < 32; ++j) {
             const int off = __shfl_sync(0xffffffffu, coff, j);
             if (row_ok && off >= 0)
               asm volatile("red.global.add.f32 [%0], %1;" ::"l"(base + off), "f"(__uint_as_float(v[j])) : "memory");
+          }
+        }
+        if (EPI == TC_DGRAD && n0 < p.N) {
+          // din[b, c, gy*s + sy, gx*s + sx] = acc[m, (sy, c, sx)]: each element exactly once, plain stores.  Lanes are
+          // consecutive block columns gx, so one store instruction covers a run of one image row per channel (s = 1: the
+          // 32 lanes write 128 contiguous bytes, like the TC_CONV NCHW output); the s = 2 pair (sx = 0, 1) of a channel
+          // sits in adjacent columns and leaves as one 8-byte store.  Lane j decodes column n0 + j once; the offsets are
+          // broadcast by shuffle.
+          const int s = p.ci_stride, sc = s * p.ci_cin;
+          const int kcol = n0 + lane;
+          int coff = -1;
+          if (kcol < p.N) {
+            const int sy = kcol / sc, r = kcol - sy * sc, c = r / s;
+            coff = (c * p.ci_h + sy) * p.ci_w + (r - c * s);
+          }
+          const bool row_ok = m < p.M;
+          const int gg = p.strip_G * p.strip_G, mm = row_ok ? m : 0;
+          const int b = mm / gg, rem = mm - b * gg, gy = rem / p.strip_G, gx = rem - gy * p.strip_G;
+          float* base = p.C + ((long)b * p.ci_cin * p.ci_h + gy * s) * p.ci_w + gx * s;
+          if (s == 2 && p.vec_acc) {
+#pragma unroll
+            for (int j = 0; j < 32; j += 2) {
+              const int off = __shfl_sync(0xffffffffu, coff, j);
+              if (row_ok && off >= 0)
+                *reinterpret_cast<float2*>(base + off) = make_float2(__uint_as_float(v[j]), __uint_as_float(v[j + 1]));
+            }
+          } else {
+#pragma unroll
+            for (int j = 0; j < 32; ++j) {
+              const int off = __shfl_sync(0xffffffffu, coff, j);
+              if (row_ok && off >= 0) base[off] = __uint_as_float(v[j]);
+            }
           }
         }
         if ((EPI == TC_STORE || EPI == TC_EMBED || (EPI == TC_BIAS_RELU && (p.M & 1) == 0) ||
@@ -843,9 +885,23 @@ int gemm_bf16_tc(int M, int N, int K, const bf16* A_hi, const bf16* A_lo, const 
   }
   if (epi == TC_EMBED) bn = 128;   // four epilogue warp sets x one 32-column chunk; 64 KB stages leave room for their staging
   // (32-wide tiles for conv3's 324 strip tiles were tried: slower -- only four epilogue warps drain a 32-column tile)
+  const bool dgrad = epi == TC_DGRAD;
+  if (dgrad) {
+    if (ex == nullptr || split3 || split2 || mn || ex->strip_t < 1 || ex->strip_G < 1 || ex->dg_cout < 8 || ex->dg_cout > 64 ||
+        ex->dg_cout % 8 || K != ex->strip_t * ex->strip_t * TBK || ex->ci_stride < 1 || ex->ci_cin < 1 ||
+        N != ex->ci_stride * ex->ci_stride * ex->ci_cin || N % 8 || M % (ex->strip_G * ex->strip_G) ||
+        ex->strip_G * ex->ci_stride > ex->ci_h || ex->strip_G * ex->ci_stride > ex->ci_w)
+      return (int)cudaErrorInvalidValue;
+    bn = N <= 64 ? 64 : N <= 128 ? 128 : 256;    // conv3: 64 columns, conv2: 128 -- one n-tile either way
+  }
   CUtensorMap ma_hi, ma_lo, mb_hi, mb_lo;
   int rc;
-  if (mn) {
+  if (dgrad) {
+    rc = make_map(&ma_hi, A_hi, M, ex->dg_cout, TBM);                                    // dYg (M, Cout)
+    if (rc) return rc;
+    rc = make_map(&mb_hi, B_hi, ex->dg_cout, (long)ex->strip_t * ex->strip_t * N, 64);   // Wd (Cout, t*t*N)
+    if (rc) return rc;
+  } else if (mn) {
     const long b_cols = ex->wg_t ? (long)ex->wg_kc * TBK : N;      // strip weight gradient: B is the block matrix
     rc = (ex->mn_major & 1) ? make_map(&ma_hi, A_hi, K, M, 64) : make_map(&ma_hi, A_hi, M, K, TBM);
     if (rc) return rc;
@@ -884,12 +940,12 @@ int gemm_bf16_tc(int M, int N, int K, const bf16* A_hi, const bf16* A_lo, const 
   p.ohw = ex ? ex->ohw : 1; p.feat = ex ? ex->feat : nullptr; p.batch = ex ? ex->batch : 1;
   p.ci_h = ex ? ex->ci_h : 0; p.ci_w = ex ? ex->ci_w : 0; p.ci_cin = ex ? ex->ci_cin : 0; p.ci_kh = ex ? ex->ci_kh : 0;
   p.ci_kw = ex ? ex->ci_kw : 0; p.ci_stride = ex ? ex->ci_stride : 0; p.ci_ow = ex ? ex->ci_ow : 0;
-  p.ci_G = ex ? ex->ci_G : 0; p.ci_oh = ex ? ex->ci_oh : 0;
   p.strip_t = ex ? ex->strip_t : 0; p.strip_G = ex ? ex->strip_G : 0; p.strip_kc = ex ? ex->strip_kc : 0;
   p.cv_oh = ex ? ex->cv_oh : 0; p.cv_ow = ex ? ex->cv_ow : 0; p.nx_s = ex ? ex->nx_s : 0; p.nx_G = ex ? ex->nx_G : 0;
   p.nx_hi = ex ? ex->nx_hi : nullptr; p.nx_lo = ex ? ex->nx_lo : nullptr;
   p.mn_major = mn ? ex->mn_major : 0; p.wg_t = ex ? ex->wg_t : 0; p.wg_G = ex ? ex->wg_G : 0; p.wg_kc = ex ? ex->wg_kc : 0;
   if (epi == TC_COL2IM && (ex == nullptr || p.ci_kh * p.ci_kw * p.ci_cin != N || split3 || split2)) return (int)cudaErrorInvalidValue;
+  if (dgrad) p.vec_acc = (reinterpret_cast<uintptr_t>(C) & 7) == 0 && (p.ci_w & 1) == 0;   // s = 2: 8-byte pair stores
   p.o_hi = ex ? ex->o_hi : nullptr; p.o_lo = ex ? ex->o_lo : nullptr;
   p.o_hiT = ex ? ex->o_hiT : nullptr; p.o_loT = ex ? ex->o_loT : nullptr;
   p.fmt = ex ? ex->fmt : 0;
@@ -936,6 +992,10 @@ int gemm_bf16_tc(int M, int N, int K, const bf16* A_hi, const bf16* A_lo, const 
     switch (epi) {
       case TC_STORE: RIQN_TC_NARROW(1, TC_STORE); RIQN_TC_GO(1, TC_STORE);
       case TC_COL2IM: RIQN_TC_GO(1, TC_COL2IM);
+      case TC_DGRAD:
+        if (bn == 64) return launch_tc<1, TC_DGRAD, 64>(ma_hi, ma_lo, mb_hi, mb_lo, p, s);
+        if (bn == 128) return launch_tc<1, TC_DGRAD, 128>(ma_hi, ma_lo, mb_hi, mb_lo, p, s);
+        RIQN_TC_GO(1, TC_DGRAD);
       case TC_BIAS_RELU: RIQN_TC_GO(1, TC_BIAS_RELU);
       case TC_ATOMIC: RIQN_TC_NARROW(1, TC_ATOMIC); RIQN_TC_GO(1, TC_ATOMIC);
       case TC_NOISY_WGRAD: RIQN_TC_GO(1, TC_NOISY_WGRAD);
