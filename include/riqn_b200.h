@@ -227,7 +227,9 @@ int riqn_quantile_embed_bwd_tc(int batch, int num_quantiles, int embed_dim, int 
 /* ------------------------------------------------------------------------------------------------
  * z-layers + dueling aggregation                          replaces rainbowiqn/model.py:153-156
  * ---------------------------------------------------------------------------------------------- */
-/* h (rows, 2*hidden) = [value-stream hidden | advantage-stream hidden]; wz (1+A, hidden) = effective
+/* Domain of the three dueling entry points: hidden in {128, 256, ..., 1024} (a multiple of 128), 1 <= A <= 31, and the
+ * shared memory of the kernel the call selects within 227 KB; anything else returns cudaErrorInvalidValue before a launch.
+ * h (rows, 2*hidden) = [value-stream hidden | advantage-stream hidden]; wz (1+A, hidden) = effective
  * weights of fcnoisy_z_v (row 0) and fcnoisy_z_a; bz (1+A).  q (rows, A) = v + a - mean_a a. */
 int riqn_dueling_fwd(long rows, int batch, int hidden, int action_space, const float* h, const float* wz,
                      const float* bz, float* q, void* stream);
@@ -243,7 +245,9 @@ int riqn_dueling_bwd(long rows, int batch, int hidden, int action_space, const f
  * as bf16 (and its transpose dh_hi_t (2*hidden, rows) if non-NULL), dh_colsum (2*hidden) = the fp32 column sums of dh
  * (zeroed here; pass it to riqn_noisy_bias_grad with dh == NULL) and dz_bf16 (rows, 32), if non-NULL, the bf16 image of
  * dz for riqn_z_wgrad_tc.  Only the sign of h matters here (ReLU mask): h_bf16 (rows, 2*hidden), if non-NULL, is read
- * instead of h. */
+ * instead of h.  The transposed image needs a 32 x 2*hidden bf16 tile (128*hidden bytes) beside the
+ * ((1+A)*hidden + 3*hidden) floats of the weights and sums; where that exceeds 227 KB (e.g. hidden 1024 with A = 24) a
+ * non-NULL dh_hi_t is refused. */
 int riqn_dueling_bwd_bf16(long rows, int batch, int hidden, int action_space, const float* h, const void* h_bf16,
                           const float* wz,
                           const float* dtheta, const float* gscale, float gscale_mul, const long long* actions, void* dh_hi,

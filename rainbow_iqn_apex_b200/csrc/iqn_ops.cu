@@ -433,10 +433,17 @@ __global__ void z_dueling_fwd_kernel(long R, int B, int A, const float* __restri
 // of a thread are in flight together, and the four dot products of one output are reduced with 6 shuffles (a
 // transpose-reduce over lane bits 4 and 3, then a butterfly over bits 2..0): lane l ends up with the sums of row
 // rr(l) = 2*bit3(l) + bit4(l), and the 8 lanes of a row share out the A advantages.
+// The row registers hx[4][HID/128] are 16*HID/128 floats: up to 512 they fit two blocks per SM (128-register cap); wider
+// layers run one block per SM so that nothing spills.
 template <int HID>
-__global__ void __launch_bounds__(256, 2) z_dueling_fwd4_kernel(long R, int B, int A, const float* __restrict__ H,
-                                                                const float* __restrict__ Wz, const float* __restrict__ bz,
-                                                                float* __restrict__ q) {
+constexpr int zd_fwd4_min_blocks() { return HID <= 512 ? 2 : 1; }
+
+template <int HID>
+__global__ void __launch_bounds__(256, zd_fwd4_min_blocks<HID>()) z_dueling_fwd4_kernel(long R, int B, int A,
+                                                                                        const float* __restrict__ H,
+                                                                                        const float* __restrict__ Wz,
+                                                                                        const float* __restrict__ bz,
+                                                                                        float* __restrict__ q) {
   extern __shared__ float sW[];  // (1+A) * HID
   for (int i = threadIdx.x; i < (1 + A) * HID / 4; i += blockDim.x)
     reinterpret_cast<float4*>(sW)[i] = reinterpret_cast<const float4*>(Wz)[i];
@@ -515,8 +522,8 @@ __global__ void __launch_bounds__(256, 2) z_dueling_fwd4_kernel(long R, int B, i
 // Every warp owns one 4-row stage (4 x 2*HID floats, contiguous in H) filled by a bulk async copy that completes on the
 // warp's mbarrier; as soon as the advantage halves of the current rows sit in registers, lane 0 launches the copy of the
 // warp's next 4 rows, which then runs under the A advantage products (95 % of the arithmetic).  The row registers are no
-// longer the only bytes in flight, so one CTA of 8 warps per SM keeps HBM busy, and with the register cap gone the
-// advantage loop runs two independent product / shuffle chains at a time.
+// longer the only bytes in flight, so one CTA per SM (zs_warps: 8 warps at HID = 512) keeps HBM busy, and with the
+// register cap gone the advantage loop runs two independent product / shuffle chains at a time.
 __device__ __forceinline__ uint32_t zs_smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
 __device__ __forceinline__ void zs_bulk_load(void* dst, const void* src, uint32_t bytes, uint64_t* bar) {
   asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(zs_smem_u32(bar)), "r"(bytes) : "memory");
@@ -539,17 +546,22 @@ __device__ __forceinline__ void zs_wait(uint64_t* bar, uint32_t parity) {
       : "memory");
 }
 
-constexpr int ZS_WARPS = 8;
+// Warps per CTA: as many 4-row stages as fit in 128 KB (8 at HID = 512), at most 16.  The bytes in flight per SM stay at
+// 128 KB for every width from 256 up, and the z-weights keep room beside them.
+template <int HID>
+constexpr int zs_warps() { return 4096 / HID < 16 ? 4096 / HID : 16; }
 template <int HID>
 constexpr size_t zs_smem_bytes(int A) {
-  return (size_t)ZS_WARPS * 4 * 2 * HID * sizeof(float) + (size_t)(1 + A) * HID * sizeof(float) + 32 * sizeof(float) +
-         ZS_WARPS * sizeof(uint64_t);
+  return (size_t)zs_warps<HID>() * 4 * 2 * HID * sizeof(float) + (size_t)(1 + A) * HID * sizeof(float) + 32 * sizeof(float) +
+         zs_warps<HID>() * sizeof(uint64_t);
 }
 
 template <int HID>
-__global__ void __launch_bounds__(ZS_WARPS * 32, 1) z_dueling_fwd4s_kernel(long R, int B, int A, const float* __restrict__ H,
-                                                                          const float* __restrict__ Wz,
-                                                                          const float* __restrict__ bz, float* __restrict__ q) {
+__global__ void __launch_bounds__(zs_warps<HID>() * 32, 1) z_dueling_fwd4s_kernel(long R, int B, int A,
+                                                                                 const float* __restrict__ H,
+                                                                                 const float* __restrict__ Wz,
+                                                                                 const float* __restrict__ bz, float* __restrict__ q) {
+  constexpr int ZS_WARPS = zs_warps<HID>();
   extern __shared__ __align__(1024) unsigned char zs_raw[];
   constexpr int ROW = 2 * HID;                                  // floats per row of H
   float* stage_all = reinterpret_cast<float*>(zs_raw);          // ZS_WARPS x (4 rows)
@@ -781,8 +793,9 @@ __global__ void z_dueling_bwd_kernel(long R, int B, int A, const float* __restri
 
 // bf16-operand variant: the data gradient leaves directly as the two bf16 images the tensor-core products consume
 // (dh_hi (R, 2*HID) for the dgrad, dh_hiT (2*HID, R) for the wgrad) plus its fp32 column sums (bias gradients); the fp32
-// dH matrix is never written.  One block = 32 consecutive rows; the transposed image goes through an XOR-swizzled
-// shared tile (16-byte chunk c/8 of row r sits in slot (c/8) ^ ((r >> 3) & 3)) and leaves as 64-byte column segments.
+// dH matrix is never written.  One block = 32 consecutive rows; a row is 2*HID/8 chunks of 8 columns, HC = HID/128 per
+// lane.  The transposed image goes through an XOR-swizzled shared tile (16-byte chunk c/8 of row r sits in slot
+// (c/8) ^ ((r >> 3) & 3)) and leaves as 64-byte column segments; the tile exists only when dh_hiT is requested.
 template <int HID>
 __global__ void __launch_bounds__(256) z_dueling_bwd_bf16_kernel(long R, int B, int A, const float* __restrict__ H,
                                                                  const __nv_bfloat16* __restrict__ Hb,
@@ -794,10 +807,12 @@ __global__ void __launch_bounds__(256) z_dueling_bwd_bf16_kernel(long R, int B, 
                                                                  __nv_bfloat16* __restrict__ dh_hiT,
                                                                  float* __restrict__ colsum, float* __restrict__ dz,
                                                                  __nv_bfloat16* __restrict__ dz_bf) {
+  constexpr int HC = HID / 128;                        // 8-column chunks per lane and row
+  constexpr int NCH = 2 * HID / 8;                     // chunks per row
   extern __shared__ __align__(16) float sW[];          // (1+A)*HID weights | HID colmean | 2*HID column sums | tile
   float* wbar = sW + (1 + A) * HID;
   float* cs = wbar + HID;
-  uint4* tile = reinterpret_cast<uint4*>(cs + 2 * HID);   // [32 rows][128 chunks of 8 bf16]
+  uint4* tile = reinterpret_cast<uint4*>(cs + 2 * HID);   // [32 rows][NCH chunks of 8 bf16], only if dh_hiT != NULL
   for (int i = threadIdx.x; i < (1 + A) * HID / 4; i += blockDim.x)
     reinterpret_cast<float4*>(sW)[i] = reinterpret_cast<const float4*>(Wz)[i];
   for (int i = threadIdx.x; i < 2 * HID; i += blockDim.x) cs[i] = 0.f;
@@ -810,9 +825,9 @@ __global__ void __launch_bounds__(256) z_dueling_bwd_bf16_kernel(long R, int B, 
   __syncthreads();
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int Nq = (int)(R / B);
-  float bs[4][8];
+  float bs[HC][8];
 #pragma unroll
-  for (int it = 0; it < 4; ++it)
+  for (int it = 0; it < HC; ++it)
 #pragma unroll
     for (int i = 0; i < 8; ++i) bs[it][i] = 0.f;
   const long n_blk = (R + 31) / 32;
@@ -829,9 +844,9 @@ __global__ void __launch_bounds__(256) z_dueling_bwd_bf16_kernel(long R, int B, 
     const float* wa = sW + (1 + act) * HID;
     // the ReLU mask only needs the SIGN of h: read the bf16 image when the forward left one (half the bytes); all of
     // a row's loads are issued before the first use
-    float hrow[4][8];
+    float hrow[HC][8];
 #pragma unroll
-    for (int it = 0; it < 4; ++it) {
+    for (int it = 0; it < HC; ++it) {
       const int c0 = (lane + 32 * it) * 8;
 #pragma unroll
       for (int i = 0; i < 8; ++i) hrow[it][i] = 0.f;
@@ -853,14 +868,18 @@ __global__ void __launch_bounds__(256) z_dueling_bwd_bf16_kernel(long R, int B, 
       }
     }
 #pragma unroll
-    for (int it = 0; it < 4; ++it) {
-      const int chunk = lane + 32 * it, c0 = chunk * 8, j0 = c0 & (HID - 1);
+    for (int it = 0; it < HC; ++it) {
+      const int chunk = lane + 32 * it, c0 = chunk * 8;
       const float (&hv)[8] = hrow[it];
       float val[8];
-      if (it < 2) {                                            // value stream: dv * w_zv
+      // chunk group it covers columns [256*it, 256*it + 256): wholly one stream unless HID / 256 is not whole (384, 640,
+      // 896), where one group straddles the two streams and each lane picks its own
+      const bool value = (it + 1) * 256 <= HID ? true : (it * 256 >= HID ? false : c0 < HID);
+      if (value) {                                             // value stream: dv * w_zv
 #pragma unroll
-        for (int i = 0; i < 8; ++i) val[i] = hv[i] > 0.f ? g * sW[j0 + i] : 0.f;
+        for (int i = 0; i < 8; ++i) val[i] = hv[i] > 0.f ? g * sW[c0 + i] : 0.f;
       } else {                                                 // advantage stream: g * (W_za[act] - colmean)
+        const int j0 = c0 - HID;
 #pragma unroll
         for (int i = 0; i < 8; ++i) val[i] = hv[i] > 0.f ? g * (wa[j0 + i] - wbar[j0 + i]) : 0.f;
       }
@@ -874,7 +893,7 @@ __global__ void __launch_bounds__(256) z_dueling_bwd_bf16_kernel(long R, int B, 
       }
       const uint4 pk = make_uint4(w[0], w[1], w[2], w[3]);
       if (ok) *reinterpret_cast<uint4*>(dh_hi + r * (2 * HID) + c0) = pk;
-      if (dh_hiT) tile[rl * 128 + (chunk ^ ((rl >> 3) & 3))] = pk;
+      if (dh_hiT) tile[rl * NCH + (chunk ^ ((rl >> 3) & 3))] = pk;
     }
     if (ok) {
       float z = 0.f;
@@ -895,8 +914,8 @@ __global__ void __launch_bounds__(256) z_dueling_bwd_bf16_kernel(long R, int B, 
       uint32_t w[4];
 #pragma unroll
       for (int i = 0; i < 4; ++i) {
-        const unsigned short lo = t16[((8 * piece + 2 * i) * 128 + slot) * 8 + (c & 7)];
-        const unsigned short hi = t16[((8 * piece + 2 * i + 1) * 128 + slot) * 8 + (c & 7)];
+        const unsigned short lo = t16[((8 * piece + 2 * i) * NCH + slot) * 8 + (c & 7)];
+        const unsigned short hi = t16[((8 * piece + 2 * i + 1) * NCH + slot) * 8 + (c & 7)];
         w[i] = (uint32_t)lo | ((uint32_t)hi << 16);
       }
       *reinterpret_cast<uint4*>(dh_hiT + (long)c * R + r0 + 8 * piece) = make_uint4(w[0], w[1], w[2], w[3]);
@@ -905,7 +924,7 @@ __global__ void __launch_bounds__(256) z_dueling_bwd_bf16_kernel(long R, int B, 
   __syncthreads();                                               // the tile is rewritten by the next row block
   }
 #pragma unroll
-  for (int it = 0; it < 4; ++it)
+  for (int it = 0; it < HC; ++it)
 #pragma unroll
     for (int i = 0; i < 8; ++i) atomicAdd(&cs[(lane + 32 * it) * 8 + i], bs[it][i]);
   __syncthreads();
@@ -1226,57 +1245,123 @@ RIQN_API int riqn_noisy_bias_grad(long rows, int out_features, const float* dh, 
   return (int)cudaGetLastError();
 }
 
+// ------------------------------------------------------------------------------------------------
+// z-layer + dueling entry points: one instantiation per supported width (every multiple of 128 up to 1024), each with
+// its own per-device attribute cache.  A (width, A) pair whose shared memory does not fit is refused before any launch.
+// ------------------------------------------------------------------------------------------------
+namespace riqn {
+constexpr size_t kMaxSmemOptin = 227 * 1024;   // opt-in dynamic shared memory per block on sm_100a
+
+static inline bool hidden_supported(int hidden) { return hidden >= 128 && hidden <= 1024 && hidden % 128 == 0; }
+
+static inline size_t dueling_bwd_bf16_smem(int hidden, int A, bool transposed) {
+  return sizeof(float) * ((size_t)(1 + A) * hidden + hidden + 2 * hidden) + (transposed ? (size_t)32 * (2 * hidden / 8) * 16 : 0);
+}
+
+template <int HID>
+static int dueling_fwd_launch(long rows, int batch, int A, const float* h, const float* wz, const float* bz, float* q,
+                              cudaStream_t s) {
+  const size_t smem = sizeof(float) * (1 + A) * HID;
+  const int dev = PerDeviceOnce::device();
+  if (A <= 24) {
+    if (rows >= 4096 && (reinterpret_cast<uintptr_t>(h) & 15) == 0 && zs_smem_bytes<HID>(A) <= kMaxSmemOptin) {
+      static PerDeviceOnce attrs_once;                                       // streamed variant: one CTA per SM
+      if (!attrs_once.done[dev]) {
+        const size_t most = zs_smem_bytes<HID>(24) < kMaxSmemOptin ? zs_smem_bytes<HID>(24) : kMaxSmemOptin;
+        RIQN_CUDA(cudaFuncSetAttribute(z_dueling_fwd4s_kernel<HID>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)most));
+        attrs_once.done[dev] = true;
+      }
+      z_dueling_fwd4s_kernel<HID><<<148, zs_warps<HID>() * 32, zs_smem_bytes<HID>(A), s>>>(rows, batch, A, h, wz, bz, q);
+      return (int)cudaGetLastError();
+    }
+    static PerDeviceOnce attr4_once;
+    if (!attr4_once.done[dev]) {
+      RIQN_CUDA(cudaFuncSetAttribute(z_dueling_fwd4_kernel<HID>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                     (int)(sizeof(float) * 25 * HID)));
+      attr4_once.done[dev] = true;
+    }
+    z_dueling_fwd4_kernel<HID><<<148 * 2, 256, smem, s>>>(rows, batch, A, h, wz, bz, q);
+  } else {
+    static PerDeviceOnce attr_once;
+    if (!attr_once.done[dev]) {
+      RIQN_CUDA(cudaFuncSetAttribute(z_dueling_fwd_kernel<HID>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                     (int)(sizeof(float) * 32 * HID)));
+      attr_once.done[dev] = true;
+    }
+    z_dueling_fwd_kernel<HID><<<148 * 4, 256, smem, s>>>(rows, batch, A, h, wz, bz, q);
+  }
+  return (int)cudaGetLastError();
+}
+
+template <int HID>
+static int dueling_bwd_launch(long rows, int batch, int A, const float* h, const float* wz, const float* dtheta,
+                              const float* gscale, float gscale_mul, const long long* actions, float* dh, float* dz,
+                              void* dz_bf16, cudaStream_t s) {
+  const size_t smem = sizeof(float) * ((1 + A) * HID + HID);
+  static PerDeviceOnce attr_once;
+  const int dev = PerDeviceOnce::device();
+  if (!attr_once.done[dev]) {
+    RIQN_CUDA(cudaFuncSetAttribute(z_dueling_bwd_kernel<HID>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                   (int)(sizeof(float) * 33 * HID)));
+    attr_once.done[dev] = true;
+  }
+  z_dueling_bwd_kernel<HID><<<148 * 4, 256, smem, s>>>(rows, batch, A, h, wz, dtheta, gscale, gscale_mul,
+                                                        (const int64_t*)actions, dh, dz, (__nv_bfloat16*)dz_bf16);
+  return (int)cudaGetLastError();
+}
+
+template <int HID>
+static int dueling_bwd_bf16_launch(long rows, int batch, int A, const float* h, const void* h_bf16, const float* wz,
+                                   const float* dtheta, const float* gscale, float gscale_mul, const long long* actions,
+                                   void* dh_hi, void* dh_hi_t, float* dh_colsum, float* dz, void* dz_bf16, cudaStream_t s) {
+  const size_t smem = dueling_bwd_bf16_smem(HID, A, dh_hi_t != nullptr);
+  static PerDeviceOnce attr_once;
+  const int dev = PerDeviceOnce::device();
+  if (!attr_once.done[dev]) {
+    const size_t most = dueling_bwd_bf16_smem(HID, 31, true) < kMaxSmemOptin ? dueling_bwd_bf16_smem(HID, 31, true) : kMaxSmemOptin;
+    RIQN_CUDA(cudaFuncSetAttribute(z_dueling_bwd_bf16_kernel<HID>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)most));
+    attr_once.done[dev] = true;
+  }
+  RIQN_CUDA(cudaMemsetAsync(dh_colsum, 0, sizeof(float) * 2 * HID, s));
+  const long n_blk = (rows + 31) / 32;
+  z_dueling_bwd_bf16_kernel<HID><<<(unsigned)(n_blk < 148 * 2 ? n_blk : 148 * 2), 256, smem, s>>>(
+      rows, batch, A, h, (const __nv_bfloat16*)h_bf16, wz, dtheta, gscale, gscale_mul, (const int64_t*)actions,
+      (__nv_bfloat16*)dh_hi, (__nv_bfloat16*)dh_hi_t, dh_colsum, dz, (__nv_bfloat16*)dz_bf16);
+  return (int)cudaGetLastError();
+}
+}  // namespace riqn
+
+#define RIQN_HIDDEN_DISPATCH(hidden, launch, ...)                                                                       \
+  switch (hidden) {                                                                                                    \
+    case 128: return launch<128>(__VA_ARGS__);                                                                         \
+    case 256: return launch<256>(__VA_ARGS__);                                                                         \
+    case 384: return launch<384>(__VA_ARGS__);                                                                         \
+    case 512: return launch<512>(__VA_ARGS__);                                                                         \
+    case 640: return launch<640>(__VA_ARGS__);                                                                         \
+    case 768: return launch<768>(__VA_ARGS__);                                                                         \
+    case 896: return launch<896>(__VA_ARGS__);                                                                         \
+    case 1024: return launch<1024>(__VA_ARGS__);                                                                       \
+    default: return (int)cudaErrorInvalidValue;                                                                        \
+  }
+
 RIQN_API int riqn_dueling_fwd(long rows, int batch, int hidden, int action_space, const float* h, const float* wz,
                               const float* bz, float* q, void* stream) {
   riqn::note_launches(1);
-  if (hidden != 512 || action_space > 31) return (int)cudaErrorInvalidValue;
-  const size_t smem = sizeof(float) * (1 + action_space) * hidden;
-  static PerDeviceOnce attr_once;
-  const int attr_dev = PerDeviceOnce::device();
-  if (!attr_once.done[attr_dev]) {
-    RIQN_CUDA(cudaFuncSetAttribute(z_dueling_fwd_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
-    attr_once.done[attr_dev] = true;
-  }
-  if (action_space <= 24) {
-    static PerDeviceOnce attr4_once;
-    const int attr4_dev = PerDeviceOnce::device();
-    if (!attr4_once.done[attr4_dev]) {
-      RIQN_CUDA(cudaFuncSetAttribute(z_dueling_fwd4_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
-      attr4_once.done[attr4_dev] = true;
-    }
-    if (rows >= 4096 && (reinterpret_cast<uintptr_t>(h) & 15) == 0) {      // streamed variant: one CTA per SM
-      static PerDeviceOnce attrs_once;
-      if (!attrs_once.done[attr4_dev]) {
-        RIQN_CUDA(cudaFuncSetAttribute(z_dueling_fwd4s_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                       (int)zs_smem_bytes<512>(24)));
-        attrs_once.done[attr4_dev] = true;
-      }
-      z_dueling_fwd4s_kernel<512><<<148, ZS_WARPS * 32, zs_smem_bytes<512>(action_space), (cudaStream_t)stream>>>(
-          rows, batch, action_space, h, wz, bz, q);
-      return (int)cudaGetLastError();
-    }
-    z_dueling_fwd4_kernel<512><<<148 * 2, 256, smem, (cudaStream_t)stream>>>(rows, batch, action_space, h, wz, bz, q);
-  } else {
-    z_dueling_fwd_kernel<512><<<148 * 4, 256, smem, (cudaStream_t)stream>>>(rows, batch, action_space, h, wz, bz, q);
-  }
-  return (int)cudaGetLastError();
+  if (!hidden_supported(hidden) || action_space < 1 || action_space > 31 ||
+      sizeof(float) * (1 + action_space) * hidden > kMaxSmemOptin)
+    return (int)cudaErrorInvalidValue;
+  RIQN_HIDDEN_DISPATCH(hidden, dueling_fwd_launch, rows, batch, action_space, h, wz, bz, q, (cudaStream_t)stream);
 }
 
 RIQN_API int riqn_dueling_bwd(long rows, int batch, int hidden, int action_space, const float* h, const float* wz,
                               const float* dtheta, const float* gscale, float gscale_mul, const long long* actions, float* dh, float* dz,
                               void* dz_bf16, void* stream) {
   riqn::note_launches(1);
-  if (hidden != 512 || action_space > 31) return (int)cudaErrorInvalidValue;
-  const size_t smem = sizeof(float) * ((1 + action_space) * hidden + hidden);
-  static PerDeviceOnce attr_once;
-  const int attr_dev = PerDeviceOnce::device();
-  if (!attr_once.done[attr_dev]) {
-    RIQN_CUDA(cudaFuncSetAttribute(z_dueling_bwd_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024));
-    attr_once.done[attr_dev] = true;
-  }
-  z_dueling_bwd_kernel<512><<<148 * 4, 256, smem, (cudaStream_t)stream>>>(rows, batch, action_space, h, wz, dtheta, gscale, gscale_mul,
-                                                                       (const int64_t*)actions, dh, dz, (__nv_bfloat16*)dz_bf16);
-  return (int)cudaGetLastError();
+  if (!hidden_supported(hidden) || action_space < 1 || action_space > 31 ||
+      sizeof(float) * ((1 + action_space) * hidden + hidden) > kMaxSmemOptin)
+    return (int)cudaErrorInvalidValue;
+  RIQN_HIDDEN_DISPATCH(hidden, dueling_bwd_launch, rows, batch, action_space, h, wz, dtheta, gscale, gscale_mul, actions, dh,
+                       dz, dz_bf16, (cudaStream_t)stream);
 }
 
 RIQN_API int riqn_dueling_bwd_bf16(long rows, int batch, int hidden, int action_space, const float* h, const void* h_bf16,
@@ -1284,23 +1369,14 @@ RIQN_API int riqn_dueling_bwd_bf16(long rows, int batch, int hidden, int action_
                                    const float* dtheta, const float* gscale, float gscale_mul, const long long* actions, void* dh_hi,
                                    void* dh_hi_t, float* dh_colsum, float* dz, void* dz_bf16, void* stream) {
   riqn::note_launches(1);
-  if (hidden != 512 || action_space > 31 || rows % 8) return (int)cudaErrorInvalidValue;
-  cudaStream_t s = (cudaStream_t)stream;
-  const size_t smem = sizeof(float) * ((1 + action_space) * hidden + hidden + 2 * hidden) + 32 * 128 * 16;
-  static PerDeviceOnce attr_once;
-  const int attr_dev = PerDeviceOnce::device();
-  if (!attr_once.done[attr_dev]) {
-    RIQN_CUDA(cudaFuncSetAttribute(z_dueling_bwd_bf16_kernel<512>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024));
-    attr_once.done[attr_dev] = true;
-  }
-  RIQN_CUDA(cudaMemsetAsync(dh_colsum, 0, sizeof(float) * 2 * hidden, s));
-  const long n_blk = (rows + 31) / 32;
-  z_dueling_bwd_bf16_kernel<512><<<(unsigned)(n_blk < 148 * 2 ? n_blk : 148 * 2), 256, smem, s>>>(
-      rows, batch, action_space, h, (const __nv_bfloat16*)h_bf16, wz, dtheta, gscale, gscale_mul, (const int64_t*)actions,
-      (__nv_bfloat16*)dh_hi,
-      (__nv_bfloat16*)dh_hi_t, dh_colsum, dz, (__nv_bfloat16*)dz_bf16);
-  return (int)cudaGetLastError();
+  // the transposed image needs a (32 rows x 2*hidden) bf16 tile beside the weights: refused where it does not fit
+  if (!hidden_supported(hidden) || action_space < 1 || action_space > 31 || rows % 8 ||
+      dueling_bwd_bf16_smem(hidden, action_space, dh_hi_t != nullptr) > kMaxSmemOptin)
+    return (int)cudaErrorInvalidValue;
+  RIQN_HIDDEN_DISPATCH(hidden, dueling_bwd_bf16_launch, rows, batch, action_space, h, h_bf16, wz, dtheta, gscale, gscale_mul,
+                       actions, dh_hi, dh_hi_t, dh_colsum, dz, dz_bf16, (cudaStream_t)stream);
 }
+#undef RIQN_HIDDEN_DISPATCH
 
 RIQN_API int riqn_z_wgrad(long rows, int hidden, int action_space, const float* dz, const float* h, float* dwz_scratch,
                           float* dbz_scratch, const float* eps_w_zv, const float* eps_b_zv, const float* eps_w_za,

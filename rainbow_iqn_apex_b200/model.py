@@ -13,6 +13,10 @@ Adam moments in matching arenas), ordered so that fcnoisy_h_v|fcnoisy_h_a form a
 are views of the arena, so torch's state_dict / load_state_dict / checkpoints keep working while the
 optimiser and the gradient all-reduce touch one contiguous buffer.
 
+Supported widths: ``hidden_size`` is any multiple of 128 up to 1024 (``HIDDEN_SIZES``).  The z-layer + dueling kernels
+are instantiated once per width; the head products take the width at run time.  Other widths raise ValueError, and so
+does an IQN action space the dueling kernels cannot hold (``check_dueling_shape``).
+
 There is no PyTorch fallback: every tensor operation below is a C-ABI call (include/riqn_b200.h).
 """
 import math
@@ -41,6 +45,33 @@ _ALIGN = 64  # floats; arena groups start on 256-byte boundaries
 PRECISION = {"fwd": os.environ.get("RIQN_FWD_PRECISION", "fp16"), "bwd": os.environ.get("RIQN_BWD_PRECISION", "bf16")}
 WGRAD_SPLIT_K = int(os.environ.get("RIQN_WGRAD_SPLIT_K", "4"))
 _NO_STRIP = os.environ.get("RIQN_NO_STRIP_CONV", "0") == "1"      # fall back to the explicit-im2col forward
+
+# Widths of the two hidden NoisyLinear layers with z-layer + dueling kernels: 2*hidden is then a multiple of 256 (whole
+# head-product n-tiles) and every lane of the dueling kernels owns whole float4 / 8-wide bf16 chunks.
+HIDDEN_SIZES = tuple(range(128, 1025, 128))
+MAX_DUELING_ACTIONS = 31          # the dueling kernels keep one advantage per lane (lane 0 holds the value)
+SMEM_PER_BLOCK = 227 * 1024       # opt-in dynamic shared memory per block on sm_100a
+
+
+def dueling_smem_bytes(hidden, action_space):
+    """Largest dynamic shared memory the IQN head's z-layer + dueling kernels need for (hidden, A) on the learner path:
+    the (1+A, hidden) z-weights, plus the advantage column means and the 2*hidden column sums of the backward."""
+    return 4 * max((1 + action_space) * hidden,             # riqn_dueling_fwd
+                   (1 + action_space) * hidden + hidden,    # riqn_dueling_bwd
+                   (1 + action_space) * hidden + 3 * hidden)  # riqn_dueling_bwd_bf16 (no transposed image)
+
+
+def check_dueling_shape(hidden, action_space):
+    """Raise ValueError unless the IQN head's kernels run at this (hidden, A)."""
+    if hidden not in HIDDEN_SIZES:
+        raise ValueError(f"hidden_size={hidden} is not supported: the sm_100a kernels take hidden_size in {HIDDEN_SIZES} "
+                         "(a multiple of 128 up to 1024)")
+    if not 1 <= action_space <= MAX_DUELING_ACTIONS:
+        raise ValueError(f"action_space={action_space} is not supported by the IQN dueling kernels (1..{MAX_DUELING_ACTIONS})")
+    need = dueling_smem_bytes(hidden, action_space)
+    if need > SMEM_PER_BLOCK:
+        raise ValueError(f"hidden_size={hidden} with action_space={action_space} needs {need} bytes of shared memory per "
+                         f"block in the dueling kernels; the limit is {SMEM_PER_BLOCK}")
 
 
 def set_precision(fwd=None, bwd=None):
@@ -161,7 +192,8 @@ def _geom(batch, cin, h, cout, k, stride, pad, in_bstride=None):
 
 
 class DQN(nn.Module):
-    """Reference model.py:56-162 (IQN branch; the C51 branch lives in c51.py)."""
+    """Reference model.py:56-162 (IQN branch; the C51 branch lives in c51.py).  ``args.hidden_size`` must be in
+    HIDDEN_SIZES; the IQN head also needs ``check_dueling_shape(hidden_size, action_space)`` to pass."""
 
     def __init__(self, args, action_space):
         super().__init__()
@@ -171,8 +203,11 @@ class DQN(nn.Module):
         self.disable_cuda = args.disable_cuda
         self.history = args.history_length
         self.hidden = args.hidden_size
-        if self.hidden != 512:
-            raise ValueError("the sm_100a kernels are specialised for hidden_size == 512")
+        if self.hidden not in HIDDEN_SIZES:
+            raise ValueError(f"hidden_size={self.hidden} is not supported: the sm_100a kernels take hidden_size in "
+                             f"{HIDDEN_SIZES} (a multiple of 128 up to 1024)")
+        if not self.rainbow_only:
+            check_dueling_shape(self.hidden, action_space)
         self.conv1 = nn.Conv2d(args.history_length, 32, 8, stride=4, padding=1)
         self.conv2 = nn.Conv2d(32, 64, 4, stride=2)
         self.conv3 = nn.Conv2d(64, 64, 3)
